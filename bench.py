@@ -8,6 +8,7 @@ log_prob, on synthetic data (BASELINE.md section 2): X ~ U[0,1]^{N x d}, y = sin
     python bench.py --gpus 1 --steps 10 --warmup 3            # our engine (libgpbbmm, sm_100a)
     python bench.py --impl reference --steps 2 --warmup 1     # the reference algorithm on the host CPU cores, full N
     torchrun ... bench.py --gpus N ...                        # rows of K sharded over N GPUs (strong scaling)
+    python bench.py --steps 10 --warmup 3 --dump-outputs DIR  # + what the last timed step returned, as DIR/<name>.npy
 
 Rank 0 prints ONE JSON line (see the task contract): value = whole-job MLL evals/s with inputs resident in HBM,
 e2e = same metric through the public gpytorch-style API with HOST inputs (H2D of X, y and D2H of the result
@@ -243,12 +244,12 @@ def run_reference(args, w):
         emit({"impl": "reference", "unavailable": f"dense K at N={w['n']} does not fit in this host's memory; "
               "the reference's default path materialises K (lazy_evaluated_kernel_tensor.py:343-373)"})
         return
-    # every step is ONE evaluation at the full configuration (never a scaled sample).  The requested warm-up / step counts
-    # are honoured as long as the run stays within ~5 minutes; beyond that warm-up, then steps, are cut and the line says so.
+    # every step is ONE evaluation at the full configuration (never a scaled sample).  All requested steps run; the requested
+    # warm-up count is honoured as long as the run stays within ~5 minutes, beyond that it is cut and the line says so.
     t_probe, r = cpu_reference_eval(w)            # also the first warm-up evaluation
     budget = float(os.environ.get("GP_REF_BUDGET_S", 300.0))
     warm = max(0, min(args.warmup - 1, int((budget - args.steps * t_probe) / t_probe) - 1))
-    steps = max(1, min(args.steps, int((budget - (1 + warm) * t_probe) / t_probe)))
+    steps = args.steps
     for _ in range(warm):
         cpu_reference_eval(w)
     times = []
@@ -271,11 +272,33 @@ def run_reference(args, w):
         "gpu_launches": 0,
     }
     emit(line)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"mll": r.mll, "log_prob": r.log_prob, "inv_quad": r.inv_quad, "logdet": r.logdet,
+                                         "cg_iters": r.iters})
 
 
 # ------------------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------------------
+def dump_outputs(path, arrays):
+    """--dump-outputs: one path/<name>.npy per returned value, float32 arrays as they are and everything else as float64, so
+    that runs of two builds on the same (seeded) inputs can be compared value for value."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(path, f"{name}.npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
+def mll_result_arrays(res, t, prefix=""):
+    """The fields of the MllResult Plan.mll returns; resid holds one CG residual norm per right-hand side (t of them)."""
+    out = {k: getattr(res, k) for k in ("mll", "log_prob", "inv_quad", "logdet", "logdet_precond", "cg_iters", "tridiag_size",
+                                        "precond_rank", "status_flags")}
+    out["resid"] = [float(v) for v in res.resid[:t]]
+    return {prefix + k: v for k, v in out.items()}
+
+
 MLL_KNOBS = dict(min_precond_size=2000, precond_tol=1e-3, cg_tol=1.0, max_cg_iter=1000, max_tridiag_iter=20)  # reference defaults
 
 
@@ -463,6 +486,8 @@ def run_c4(args, w):
         "clocks": clocks, "e2e": None, "gpu_launches": None, "roofline": None, "cpu_baseline": None,
     }
     emit(line)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"mll": out.detach().cpu().numpy()})
 
 
 def run_ours(args, w):
@@ -575,8 +600,8 @@ def run_ours(args, w):
         del m["ctx"], c, xd, l2_flush
         torch.cuda.empty_cache()
         w3 = WORKLOADS["c3"]
-        m3 = measure_workload(w3, args, env, steps=max(2, min(args.steps, 5)), warmup=2)
-        c3 = {"metric": METRIC, "value": m3["value"], "unit": UNIT, "ms_per_step": m3["ms_per_step"], "steps": max(2, min(args.steps, 5)),
+        m3 = measure_workload(w3, args, env, steps=args.steps, warmup=2)
+        c3 = {"metric": METRIC, "value": m3["value"], "unit": UNIT, "ms_per_step": m3["ms_per_step"], "steps": args.steps,
               "warmup": 2, "scaling": "strong", "config": result_config(w3, world, m3),
               "roofline": {k: m3["roofline"][k] for k in ("achieved", "peak", "frac", "ms_per_launch", "mufu_bound")}}
         m3["ctx"]["plan"].close()
@@ -598,6 +623,12 @@ def run_ours(args, w):
             "parity_at_config": parity, "c3": c3,
         }
         emit(line)
+        if args.dump_outputs:
+            arrays = mll_result_arrays(res, w["probes"] + 1)
+            arrays["e2e_mll"] = e2e["mll"]
+            if c3:
+                arrays.update(mll_result_arrays(m3["res"], w3["probes"] + 1, "c3_"))
+            dump_outputs(args.dump_outputs, arrays)
     if world > 1:
         dist.barrier()
         comm.close()
@@ -614,7 +645,11 @@ def main():
     ap.add_argument("--backend", default="auto", choices=["auto", "tcgen05", "simt"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-c3", action="store_true", help="skip the secondary N=200k record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (MLL, inv_quad, logdet, ...) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     w = WORKLOADS[args.workload]
     if args.impl == "reference":

@@ -4,32 +4,33 @@ code in the build container.  `gpytorch/utils/grid.py` imports only torch and is
 `gpytorch/utils/interpolation.py` imports linear_operator (absent) for two helpers it does not use inside
 `Interpolation.interpolate`, so its source is read where it lies, the two import statements are dropped and the rest is
 executed with `convert_legacy_grid` taken from the loaded grid module.  Nothing is copied into the repo.
-Output: tests/golden/ski_golden.npz (committed).  Re-run:  python tests/golden/make_golden_ski.py
+Output: tests/golden/ski_golden.npz (committed).
+Re-run:  python tests/golden/make_golden_ski.py <path to the gpytorch source tree>
 """
 import importlib.util
 import os
+import sys
 
 import numpy as np
 import torch
 
-REF = os.environ.get("GP_REFERENCE", "/root/reference")
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def load_reference():
-    spec = importlib.util.spec_from_file_location("ref_grid", f"{REF}/gpytorch/utils/grid.py")
+def load_reference(ref):
+    spec = importlib.util.spec_from_file_location("ref_grid", f"{ref}/gpytorch/utils/grid.py")
     grid = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(grid)
-    src = open(f"{REF}/gpytorch/utils/interpolation.py").read()
+    src = open(f"{ref}/gpytorch/utils/interpolation.py").read()
     keep = [ln for ln in src.splitlines()
             if not ln.startswith("from linear_operator") and not ln.startswith("from .grid")]
     ns = {"convert_legacy_grid": grid.convert_legacy_grid, "__name__": "ref_interpolation"}
-    exec(compile("\n".join(keep), f"{REF}/gpytorch/utils/interpolation.py", "exec"), ns)
+    exec(compile("\n".join(keep), f"{ref}/gpytorch/utils/interpolation.py", "exec"), ns)
     return grid, ns["Interpolation"]
 
 
-def main():
-    grid_mod, Interpolation = load_reference()
+def main(ref):
+    grid_mod, Interpolation = load_reference(ref)
     out = {}
     cases = [("d1", [20], 37), ("d2", [12, 15], 60), ("d3", [8, 9, 10], 50), ("d3c5", [100, 100, 100], 64)]
     for dt_name, dt in (("f32", torch.float32), ("f64", torch.float64)):
@@ -67,4 +68,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])

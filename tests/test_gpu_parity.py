@@ -94,29 +94,35 @@ def test_large_d_falls_back_to_simt_and_tcgen05_refuses(Plan, cuda_dev):
 
 @pytest.mark.parametrize("tag", ["a", "b", "c", "d"])
 def test_kernel_entries_match_reference_golden(Plan, cuda_dev, golden, tag):
-    """rows() / K.V against matrices produced by the reference's own RBFCovariance / MaternCovariance."""
+    """rows() / K.V against matrices produced by the reference's own RBFCovariance / MaternCovariance (the golden file holds
+    the rows `idx` of each), and against the fp64 oracle -- pinned to the same reference outputs on the CPU -- everywhere."""
     key = f"{tag}_f64"
     x1 = torch.from_numpy(golden[f"{key}_x1"])
     same = bool(golden[f"{key}_same"])
     x2 = None if same else torch.from_numpy(golden[f"{key}_x2"])
     ls = float(golden[f"{key}_ls"])
+    idx = torch.from_numpy(golden[f"{key}_rows"])
     for kind, nk in (("rbf", "rbf"), ("matern12", "mat12"), ("matern32", "mat32"), ("matern52", "mat52")):
-        Kref = torch.from_numpy(golden[f"{key}_{nk}"])
+        Kgold = torch.from_numpy(golden[f"{key}_{nk}"])
+        Kref = ok.kernel_matrix(kind, x1, x1 if same else x2, ls, 1.0, same)
         p = Plan(x1.float().to(cuda_dev), None if same else x2.float().to(cuda_dev), backend="simt").set_hypers(kind, ls, 1.0, 0.0)
-        rows = p.rows(torch.arange(x1.size(0)))
-        assert (rows.double().cpu() - Kref).abs().max().item() < 2e-6
+        rows = p.rows(torch.arange(x1.size(0))).double().cpu()
+        assert (rows - Kref).abs().max().item() < 2e-6
+        assert (rows[idx] - Kgold).abs().max().item() < 2e-6
         p.close()
         for backend in BACKENDS:
             p = Plan(x1.float().to(cuda_dev), None if same else x2.float().to(cuda_dev), backend=backend).set_hypers(kind, ls, 1.0, 0.0)
             eye = torch.eye(Kref.size(1), dtype=torch.float32)[:, :16].contiguous()
-            out = p.kmv(eye.to(cuda_dev))  # K @ I[:, :16] = first 16 columns of K
-            assert (out.double().cpu() - Kref[:, :16]).abs().max().item() < 3e-6
+            out = p.kmv(eye.to(cuda_dev)).double().cpu()  # K @ I[:, :16] = first 16 columns of K
+            assert (out - Kref[:, :16]).abs().max().item() < 3e-6
+            assert (out[idx] - Kgold[:, :16]).abs().max().item() < 3e-6
             p.close()
     # fp32 goldens: what the reference itself produces in its default dtype
     K32 = torch.from_numpy(golden[f"{tag}_f32_rbf"]).double()
+    idx32 = torch.from_numpy(golden[f"{tag}_f32_rows"])
     p = Plan(torch.from_numpy(golden[f"{tag}_f32_x1"]).to(cuda_dev),
              None if same else torch.from_numpy(golden[f"{tag}_f32_x2"]).to(cuda_dev), backend="simt").set_hypers("rbf", ls, 1.0, 0.0)
-    assert (p.rows(torch.arange(K32.size(0))).double().cpu() - K32).abs().max().item() < 1e-5
+    assert (p.rows(idx32).double().cpu() - K32).abs().max().item() < 1e-5
     p.close()
 
 
